@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (libbdepth.so through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # reference arm: the CPU implementation on host cores
+  python bench.py ... --dump-outputs DIR                   # also write a seeded sample of the counters the last e2e step delivered
+                                                           # (DIR/positions.npy, DIR/counts.npy; the sampling runs inside that step)
 
 Workload (config.workload): BASELINE configs[1], the synthetic 30x chr20 BAM (64,444,167 bp, 12,888,833 x 150 bp
 reads, seed 20, zlib level 6, 0xFF00-byte BGZF blocks) generated on the box by tools/bamgen.c.  At N > 1 GPUs
@@ -270,6 +272,32 @@ def checksum_run(h, lin0):
         return 0
     h._ck(h.L.bdepth_run_base(h.h, L.TILE_CB(cb), None))
     return acc
+
+
+DUMP_POSITIONS = 1 << 20      # 8 + 7 x 4 bytes per position: 36 MiB of .npy files
+
+
+def counter_sampler(lin0, seed=20):
+    """A tile callback for bdepth_run_base that keeps the 7 counters of a fixed, seeded, sorted sample of linear positions
+    (the same sample for every run on the same input).  Returns (positions, counts[7, n] float32, callback); positions
+    another rank delivers stay zero."""
+    import numpy as np
+    import sambamba_b200._lib as L
+    total = int(lin0[-1])
+    pos = np.sort(np.random.default_rng(seed).choice(total, size=min(DUMP_POSITIONS, total), replace=False))
+    counts = np.zeros((7, len(pos)), np.float32)         # counters stay far below 2^24: exact in float32
+
+    def cb(_user, tp):
+        t = tp.contents
+        a = int(lin0[t.ref_id]) + t.start
+        lo, hi = np.searchsorted(pos, (a, a + t.len))
+        if hi > lo:
+            src = np.ctypeslib.as_array(t.counts, shape=(6 * t.stride + t.len,))
+            off = pos[lo:hi] - a
+            for p in range(7):
+                counts[p, lo:hi] = src[p * t.stride + off]
+        return 0
+    return pos, counts, L.TILE_CB(cb)
 
 
 def oracle_checksums(path, threads):
@@ -569,7 +597,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-file", action="store_true", help="reference arm: skip the one whole-file run of the port")
     ap.add_argument("--no-verify", action="store_true", help="development only: skip the bit-exact check of the counters after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the counters the last timed end-to-end step delivered (a fixed, seeded sample of "
+                    "positions) to DIR/positions.npy and DIR/counts.npy, so that two builds can be compared output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.config != "chr20"):
+        ap.error("--dump-outputs applies to the chr20 `depth base` workload of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -592,7 +626,7 @@ def main():
         if probe["sambamba"]:
             # the real thing (BASELINE.md 3.1): `sambamba depth base -t $(nproc)` over the whole file; without -t it is serial (depth.d:1081,1154)
             nb = os.path.getsize(path)
-            n_warm = min(a.warmup, 1)           # a whole-file run of the real thing takes most of a minute: one warm-up, then as many timed runs as the launch's budget holds
+            n_warm = min(a.warmup, 1)           # a whole-file run of the real thing takes most of a minute: at most one warm-up
             for i in range(n_warm + a.steps):
                 t0 = time.time()
                 r = subprocess.run([probe["sambamba"], "depth", "base", "-t", str(threads), path, "-o", "/dev/null"], capture_output=True, text=True)
@@ -600,11 +634,9 @@ def main():
                     raise RuntimeError(f"sambamba failed (exit {r.returncode}): {r.stderr[-300:]}")
                 if i >= n_warm:
                     times.append(time.time() - t0)
-                if times and time.time() - T_PROCESS_START + 1.5 * max(times) > BENCH_BUDGET_S:
-                    break
             dt = sum(times) / len(times)
             cb = {"value": nb / 1e9 / dt, "unit": "GB/s", "cores": threads, "kind": "sambamba", "timed_runs": len(times),
-                  "sample": f"whole file ({nb / 1e6:.0f} MB), {probe['sambamba']} depth base -t {threads}; {len(times)} timed runs within the launch's time budget"}
+                  "sample": f"whole file ({nb / 1e6:.0f} MB), {probe['sambamba']} depth base -t {threads}; {len(times)} timed runs"}
         else:
             for i in range(a.warmup + a.steps):
                 cb, dt, nb, st = cpu_baseline(path, threads, a.cpu_sample_mb << 20)
@@ -740,10 +772,16 @@ def main():
     open_s = time.perf_counter() - t0
     cold_s = None
     n_w = max(1, min(a.warmup, 3))
+    if a.dump_outputs:
+        lin0 = np.concatenate([[0], np.cumsum([l for _, l in h.refs])]).astype(np.int64)
+        dump_pos, dump_counts, dump_cb = counter_sampler(lin0)
     for i in range(n_w + a.steps):
         barrier()
         t0 = time.perf_counter()
-        h.run_base(collect=False)                                   # H2D of the compressed bytes + kernels + D2H of the counters
+        if a.dump_outputs and i == n_w + a.steps - 1:
+            h._ck(h.L.bdepth_run_base(h.h, dump_cb, None))          # the last step hands its counters to the sampler
+        else:
+            h.run_base(collect=False)                               # H2D of the compressed bytes + kernels + D2H of the counters
         dt = time.perf_counter() - t0
         s2 = h.stats()
         d2h_bytes = (s2["own_hi"] - s2["own_lo"]) * 28
@@ -753,6 +791,15 @@ def main():
         if i >= n_w:
             e2e_t.append(dt)
     e2e_stats = h.stats()
+    if a.dump_outputs:
+        if dist is not None:                                        # ranks deliver disjoint positions: their samples add up
+            parts = [None] * world
+            dist.all_gather_object(parts, dump_counts)
+            dump_counts = sum(parts)
+        if rank == 0:
+            os.makedirs(a.dump_outputs, exist_ok=True)
+            np.save(os.path.join(a.dump_outputs, "positions.npy"), dump_pos.astype(np.float64))
+            np.save(os.path.join(a.dump_outputs, "counts.npy"), dump_counts)
     # ---- rows of `depth base` formatted on the GPU (SURVEY 8d: "text formatting timed as its own line"): the same pass,
     # delivered as the text PerBasePrinter would print instead of counter planes (single GPU only; host wall clock)
     text = None
@@ -849,4 +896,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True          # the bench leaves the tree it runs from untouched (no __pycache__ of the modules it imports)
     sys.exit(main())

@@ -170,11 +170,17 @@ def test_bench_own_arm_control_flow_under_the_emulation(tmp_path):
     import subprocess
     import sys
     env = dict(os.environ, BDEPTH_BENCH_DIR=str(tmp_path), BDEPTH_BENCH_UNIT_LEN="300000")
-    r = subprocess.run([sys.executable, os.path.join(helpers.ROOT, "tests", "run_bench_emul.py"), "--reads-per-unit", "15000", "--steps", "1", "--warmup", "1", "--cpu-sample-mb", "1"],
-                       capture_output=True, text=True, env=env, timeout=900)
+    r = subprocess.run([sys.executable, os.path.join(helpers.ROOT, "tests", "run_bench_emul.py"), "--reads-per-unit", "15000", "--steps", "1", "--warmup", "1", "--cpu-sample-mb", "1",
+                        "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, env=env, timeout=900)
     assert r.returncode == 0, r.stderr[-600:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["verified"] is True and line["verification"]["checksum"] == line["verification"]["oracle_checksum"]
+    # --dump-outputs: the counters of the last timed e2e step at the sampled positions (here all 300,000 of them) are the oracle's
+    import numpy as np
+    pos, counts = np.load(tmp_path / "dump" / "positions.npy"), np.load(tmp_path / "dump" / "counts.npy")
+    assert pos.dtype == np.float64 and counts.dtype == np.float32 and counts.shape == (7, 300000) and np.array_equal(pos, np.arange(300000))
+    want, _ = helpers.oracle_counts(str(next(tmp_path.glob("*.bam"))))
+    assert counts.sum() > 0 and np.array_equal(counts, want)
     assert line["metric"] == "bam_gb_per_s_depth_base" and line["unit"] == "GB/s" and line["n_gpus"] == 1 and line["gpu_launches"] > 0
     assert set(line["roofline"]) >= {"bound", "achieved", "peak", "unit", "frac", "traffic"} and line["cpu_baseline"]["kind"] == "port"
     assert line["e2e"]["h2d_bytes_per_step"] > 0 and line["e2e"]["d2h_bytes_per_step"] == 300000 * 28
