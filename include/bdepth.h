@@ -111,6 +111,7 @@ typedef struct {
     uint64_t mate_pair_columns;   /* -m: (pair, column) decisions of selectBetterMate               */
     uint64_t mate_groups;         /* -m: names with three or more overlapping reads                 */
     float ms_mates;               /* -m: km_hash + km_link + km_fix (contained in ms_coverage)      */
+    uint32_t n_sample_passes;     /* region / window runs: pipeline passes over groups of samples (1: every sample at once); 0 otherwise */
 } bdepth_stats;
 
 /* ------------------------------------------------------------------ lifecycle */
@@ -165,8 +166,17 @@ int bdepth_set_min_baseq(bdepth_t* h, uint32_t min_base_quality);
  * reads (a chain of any length) follow the reference's none/detected/fixed/past state machine; more than eight reads
  * of one name over a single position are refused (BDEPTH_ERR_ARG). */
 int bdepth_set_fix_mates(bdepth_t* h, int on);
-/* --combined (depth.d:1131): one counter set for all samples.  Default: one per @RG sample (<= 64). */
+/* --combined (depth.d:1131): one counter set for all samples.  Default: one per @RG sample.  bdepth_run_base / _run_base_text /
+ * _run_resident hold every sample's counters at once: at most 64 samples (BDEPTH_ERR_ARG beyond).  bdepth_run_regions / _run_windows
+ * take any number: see bdepth_set_samples_per_pass. */
 int bdepth_set_combined(bdepth_t* h, int combined);
+/* Region and window runs count the samples a group at a time when their counters do not fit at once: the pipeline runs once per group
+ * of consecutive samples and each run adds the statistics of its group (a read counts in the pass of its sample only; every input is
+ * read by the passes whose groups hold one of its @RG samples).  A group holds at most 64 samples, at most what the counter window
+ * leaves room for in HBM and at most n; n = 0 (the default): as many as fit, up to 64.  Several ranks take the smallest group size of
+ * any of them.  With -m every sample has to fit one pass (BDEPTH_ERR_ARG otherwise).  bdepth_stats.n_sample_passes tells how many
+ * passes a run took. */
+int bdepth_set_samples_per_pass(bdepth_t* h, uint32_t n);
 /* Restrict runs to reads overlapping these regions (any order; merged internally).  n = 0 clears.  Regions that hold no position
  * (start >= end, or start behind the reference's end) are dropped; if none is left the restriction is cleared as with n = 0 -- a host that
  * wants "nothing" for such a query (the reference prints its header only) does not run at all, as the CLI does. */
@@ -204,7 +214,9 @@ int bdepth_run_base(bdepth_t* h, bdepth_tile_cb cb, void* user);
  * behaviour is reproduced in closed form (early threshold collection when W-O does not divide W, the
  * first-occurrence quirk of reference 0, the leftovers printed under the first trailing empty reference). */
 int bdepth_run_windows(bdepth_t* h, uint32_t window, uint32_t overlap, const uint32_t* thresholds, size_t n_thresholds, bdepth_stat_cb cb, void* user);
-/* depth region: stats for the given regions, delivered in the given order. */
+/* depth region: stats for the given regions, delivered in the given order.
+ * Both: one record per (segment, sample), segments outer, samples inner; with several sample passes
+ * (bdepth_set_samples_per_pass) delivery starts when the last pass is done, in the same order. */
 int bdepth_run_regions(bdepth_t* h, const bdepth_region* regions, size_t n, const uint32_t* thresholds, size_t n_thresholds, bdepth_stat_cb cb, void* user);
 
 /* `depth base` with the row text produced on the GPU (SURVEY 8f rank 1): the rows PerBasePrinter would print

@@ -40,7 +40,8 @@ class Stats(C.Structure):
                [(n, C.c_float) for n in ("ms_h2d", "ms_inflate", "ms_scan", "ms_coverage", "ms_reduce", "ms_d2h",
                                          "ms_total_device")] + [("host_wall_ms", C.c_double), ("ms_span_device", C.c_float), ("ms_exchange", C.c_float),
                                                                  ("own_lo", C.c_uint64), ("own_hi", C.c_uint64), ("halo_bytes_sent", C.c_uint64),
-                                                                 ("mate_pairs", C.c_uint64), ("mate_pair_columns", C.c_uint64), ("mate_groups", C.c_uint64), ("ms_mates", C.c_float)]
+                                                                 ("mate_pairs", C.c_uint64), ("mate_pair_columns", C.c_uint64), ("mate_groups", C.c_uint64), ("ms_mates", C.c_float),
+                                                                 ("n_sample_passes", C.c_uint32)]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
@@ -93,6 +94,7 @@ def load_library():
     L.bdepth_set_min_baseq.argtypes = [vp, C.c_uint32]
     L.bdepth_set_fix_mates.argtypes = [vp, C.c_int]
     L.bdepth_set_combined.argtypes = [vp, C.c_int]
+    L.bdepth_set_samples_per_pass.argtypes = [vp, C.c_uint32]
     L.bdepth_set_regions.argtypes = [vp, C.POINTER(Region), C.c_size_t]
     L.bdepth_set_shard.argtypes = [vp, C.c_int, C.c_int, vp]
     L.bdepth_nccl_unique_id.argtypes = [vp]
@@ -121,7 +123,7 @@ def load_library():
 EXPORTED_SYMBOLS = [
     "bdepth_device_count", "bdepth_open", "bdepth_open_lazy", "bdepth_open_memory", "bdepth_add_input", "bdepth_close", "bdepth_last_error", "bdepth_n_ref",
     "bdepth_ref_name", "bdepth_ref_length", "bdepth_header_text", "bdepth_is_coordinate_sorted", "bdepth_has_index",
-    "bdepth_n_samples", "bdepth_sample_name", "bdepth_set_filter", "bdepth_set_filter_query", "bdepth_set_min_baseq", "bdepth_set_fix_mates", "bdepth_set_combined", "bdepth_set_regions",
+    "bdepth_n_samples", "bdepth_sample_name", "bdepth_set_filter", "bdepth_set_filter_query", "bdepth_set_min_baseq", "bdepth_set_fix_mates", "bdepth_set_combined", "bdepth_set_samples_per_pass", "bdepth_set_regions",
     "bdepth_set_shard", "bdepth_nccl_unique_id", "bdepth_plan_shards", "bdepth_plan_region_chunks", "bdepth_set_tuning", "bdepth_stage", "bdepth_run_resident", "bdepth_run_base", "bdepth_run_base_text",
     "bdepth_run_windows", "bdepth_run_regions", "bdepth_get_stats", "bdepth_ref_has_reads", "bdepth_inflate_to_host", "bdepth_scan_to_host", "bdepth_build_index",
 ]
@@ -225,6 +227,10 @@ class BDepth:
 
     def set_combined(self, on=True):
         self._ck(self.L.bdepth_set_combined(self.h, 1 if on else 0))
+
+    def set_samples_per_pass(self, n=0):
+        """Region / window runs: count at most n samples per pipeline pass (0: as many as fit, up to 64)."""
+        self._ck(self.L.bdepth_set_samples_per_pass(self.h, n))
 
     def set_regions(self, regions):
         arr = (Region * max(1, len(regions)))(*[Region(*r) for r in regions])

@@ -160,7 +160,10 @@ struct bdepth {
     bool has_fprog = false; FilterProg fprog; DevBuf fprog_d;      // -F: compiled query (filter.cuh); otherwise mapq_gt / flag_reject
     DevBuf m_hash, m_flag, m_flt, m_ctl;
     uint32_t S = 1;                       // counter sets in the current run (samples, or 1)
-    DevBuf rg_ids, rg_offs, rg_samp;
+    uint32_t samples_per_pass = 0;        // bdepth_set_samples_per_pass: region / window runs hold at most this many samples' counters at once (0: as many as fit, up to 64)
+    uint32_t pass_g0 = 0, pass_n = 0;     // a sample pass (run_segments): the run counts samples [pass_g0, pass_g0 + pass_n) only; pass_n == 0: every sample at once
+    bool pass_untagged = false;           // set by a sample pass that met passing reads without an RG tag while it did not hold sample 0
+    DevBuf rg_ids, rg_offs, rg_samp, rg_hash, rg_tab;
     DevBuf text[2], text_tiles, text_offs, text_zero, text_samp, present;
     int coll_pending = 0;                 // several ranks: collectives of the current run this rank has not joined yet (2: the sparse decision and the boundary table; 1: the boundary table) -- a rank that stops with an error joins them with a "failed" mark, so that the others stop too instead of waiting for it
     bool want_presence = false;           // -a with -q and a positive minimum coverage: mark the positions reads cover (k_presence)
@@ -689,8 +692,12 @@ int run_pipeline_body(bdepth* h, RunMode mode, RunOut* ro, Emitter* em) {
             h->cnt_base = lo / TILE_POS * TILE_POS;
             h->win_len = ((hi - h->cnt_base + TILE_POS - 1) / TILE_POS + 1) * TILE_POS;
         }
-        h->S = (h->combined || h->hdr.sample_names.size() <= 1) ? 1u : (uint32_t)h->hdr.sample_names.size();
-        if (h->S > 64) return fail(h, BDEPTH_ERR_ARG, "%u samples: per-sample output supports at most 64 (use --combined)", h->S);
+        if (h->pass_n) h->S = h->pass_n;
+        else {
+            h->S = (h->combined || h->hdr.sample_names.size() <= 1) ? 1u : (uint32_t)h->hdr.sample_names.size();
+            // (region and window runs with more samples count them a group at a time, run_segments)
+            if (h->S > 64) return fail(h, BDEPTH_ERR_ARG, "%u samples: per-base output holds every sample's counters at once and supports at most 64 (use --combined, or depth region / depth window, which take any number of samples)", h->S);
+        }
         size_t need = (size_t)h->win_len * N_PLANES * 4 * h->S;
         size_t free_b = 0, tot_b = 0; CK(cudaMemGetInfo(&free_b, &tot_b));
         if (need > h->counts.cap && need > free_b + h->counts.cap) return fail(h, BDEPTH_ERR_CUDA, "counter window needs %zu bytes of HBM, %zu free", need, free_b);
@@ -702,15 +709,31 @@ int run_pipeline_body(bdepth* h, RunMode mode, RunOut* ro, Emitter* em) {
     CK(h->scan_stats.ensure(sizeof(ScanStats)));
     const FilterProg* d_fprog = nullptr;
     if (h->has_fprog) { CK(h->fprog_d.ensure(sizeof(FilterProg))); CK(cudaMemcpyAsync(h->fprog_d.p, &h->fprog, sizeof(FilterProg), cudaMemcpyHostToDevice, sm)); CK(cudaStreamSynchronize(sm)); d_fprog = h->fprog_d.as<FilterProg>(); }
-    RgTable rgt{nullptr, nullptr, nullptr, 0};
-    if (mode == RUN_FULL && (h->S > 1 || (fix && h->hdr.sample_names.size() > 1))) {      // @RG ID -> sample table for the per-read RG lookup (depth.d:240-250); mates pair within a sample
-        std::vector<uint8_t> ids; std::vector<uint32_t> offs; std::vector<uint8_t> samp;
-        for (size_t g = 0; g < h->hdr.rg_ids.size(); g++) { offs.push_back((uint32_t)ids.size()); ids.insert(ids.end(), h->hdr.rg_ids[g].begin(), h->hdr.rg_ids[g].end()); ids.push_back(0); samp.push_back((uint8_t)h->hdr.rg_sample[g]); }
-        CK(h->rg_ids.ensure(ids.size() + 8)); CK(h->rg_offs.ensure(offs.size() * 4 + 8)); CK(h->rg_samp.ensure(samp.size() + 8));
-        CK(cudaMemcpyAsync(h->rg_ids.p, ids.data(), ids.size(), cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(h->rg_offs.p, offs.data(), offs.size() * 4, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(h->rg_samp.p, samp.data(), samp.size(), cudaMemcpyHostToDevice, sm));
+    RgTable rgt{nullptr, nullptr, nullptr, nullptr, 0, 0, 0};
+    h->pass_untagged = false;
+    if (mode == RUN_FULL && (h->S > 1 || h->pass_n || (fix && h->hdr.sample_names.size() > 1))) {      // @RG ID -> sample table for the per-read RG lookup (depth.d:240-250); mates pair within a sample
+        // a sample pass maps the read groups of its samples to pass-local ids and every other one to RG_OTHER
+        auto local = [&](uint32_t s) -> uint16_t { return !h->pass_n ? (uint16_t)s : s - h->pass_g0 < h->pass_n ? (uint16_t)(s - h->pass_g0) : RG_OTHER; };
+        const size_t n_rg = h->hdr.rg_ids.size();
+        if (n_rg >= RG_OTHER) return fail(h, BDEPTH_ERR_ARG, "%zu read groups: at most %u are supported", n_rg, (unsigned)RG_OTHER - 1);
+        std::vector<uint8_t> ids; std::vector<uint32_t> offs; std::vector<uint16_t> samp;
+        for (size_t g = 0; g < n_rg; g++) { offs.push_back((uint32_t)ids.size()); ids.insert(ids.end(), h->hdr.rg_ids[g].begin(), h->hdr.rg_ids[g].end()); ids.push_back(0); samp.push_back(local((uint32_t)h->hdr.rg_sample[g])); }
+        uint32_t slots = 2; while (slots < 2 * n_rg) slots *= 2;
+        std::vector<uint32_t> tab(slots, 0);
+        for (size_t g = 0; g < n_rg; g++) {      // (an ID that occurs twice keeps its first line, as the linear scan it replaces did)
+            const std::string& id = h->hdr.rg_ids[g]; uint32_t hs = FNV1A_INIT; for (char c : id) hs = fnv1a_step(hs, (uint8_t)c);
+            uint32_t k = hs & (slots - 1);
+            while (tab[k] && h->hdr.rg_ids[tab[k] - 1] != id) k = (k + 1) & (slots - 1);
+            if (!tab[k]) tab[k] = (uint32_t)g + 1;
+        }
+        CK(h->rg_ids.ensure(ids.size() + 8)); CK(h->rg_offs.ensure(offs.size() * 4 + 8)); CK(h->rg_samp.ensure(samp.size() * 2 + 8)); CK(h->rg_hash.ensure(slots * 4));
+        if (n_rg) { CK(cudaMemcpyAsync(h->rg_ids.p, ids.data(), ids.size(), cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(h->rg_offs.p, offs.data(), offs.size() * 4, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(h->rg_samp.p, samp.data(), samp.size() * 2, cudaMemcpyHostToDevice, sm)); }
+        CK(cudaMemcpyAsync(h->rg_hash.p, tab.data(), slots * 4, cudaMemcpyHostToDevice, sm));
+        rgt = RgTable{h->rg_ids.as<uint8_t>(), h->rg_offs.as<uint32_t>(), h->rg_samp.as<uint16_t>(), h->rg_hash.as<uint32_t>(), slots - 1, (uint32_t)n_rg, local(0)};
+        CK(h->rg_tab.ensure(sizeof(RgTable))); CK(cudaMemcpyAsync(h->rg_tab.p, &rgt, sizeof(RgTable), cudaMemcpyHostToDevice, sm));
         CK(cudaStreamSynchronize(sm));
-        rgt = RgTable{h->rg_ids.as<uint8_t>(), h->rg_offs.as<uint32_t>(), h->rg_samp.as<uint8_t>(), (uint32_t)offs.size()};
     }
+    const RgTable* d_rgt = rgt.n_rg ? h->rg_tab.as<RgTable>() : nullptr;
     { uint64_t shard_u = blk_hi > blk_lo ? B[blk_hi - 1].uoff + B[blk_hi - 1].isize - B[blk_lo].uoff : 0; CK(h->ubuf.ensure(CARRY_MAX + std::min<uint64_t>(eff_batch_u + 65536, shard_u) + 256)); }
     CK(h->misc.ensure(64));
     HostScratch& hs = h->hs;
@@ -1039,18 +1062,20 @@ int run_pipeline_body(bdepth* h, RunMode mode, RunOut* ro, Emitter* em) {
             }
             has_dst = h->ref_has_all.as<uint32_t>();
         }
-#define K2_DECODE(F, G) BD_LAUNCH((unsigned)((nb * 32 + 255) / 256), 256, 0, sm, k2_decode<F, G>)(sp, h->chunk_start.as<int64_t>(), (uint32_t)nb, h->slot_base.as<uint32_t>(), h->slots.as<uint16_t>(), h->count.as<uint32_t>(), h->rec_base.as<uint32_t>(), soa, h->mapq_gt, h->flag_reject, h->scan_stats.as<ScanStats>(), h->long_list.as<uint32_t>(), has_dst, rgt, d_fprog, ghost_below, own_lo, own_hi, zone_below)
+#define K2_DECODE(F, G) do { if (d_rgt) K2_DECODE_RG(F, G, true); else K2_DECODE_RG(F, G, false); } while (0)
+#define K2_DECODE_RG(F, G, R) BD_LAUNCH((unsigned)((nb * 32 + 255) / 256), 256, 0, sm, k2_decode<F, G, R>)(sp, h->chunk_start.as<int64_t>(), (uint32_t)nb, h->slot_base.as<uint32_t>(), h->slots.as<uint16_t>(), h->count.as<uint32_t>(), h->rec_base.as<uint32_t>(), soa, h->mapq_gt, h->flag_reject, h->scan_stats.as<ScanStats>(), h->long_list.as<uint32_t>(), has_dst, d_rgt, d_fprog, ghost_below, own_lo, own_hi, zone_below)
         if (fix) { if (d_fprog) K2_DECODE(true, true); else K2_DECODE(false, true); }
         else if (d_fprog) K2_DECODE(true, false);
         else K2_DECODE(false, false);
 #undef K2_DECODE
+#undef K2_DECODE_RG
         CK(cudaGetLastError()); st.gpu_launches++;
         if (R && mode != RUN_INDEX && mode != RUN_SCAN_ONLY) {      // quirk 1: CIGARs that begin with N, rewritten to what the reference's cursor makes of them (the index and the raw scan see the file as it is)
             // region mode proper (no window slots, no -m, one rank): the statistics of such a read are reproduced (kernels.cuh); otherwise refused
             const bool lead_n_regions = h->seg.on && h->seg.n && !h->seg.has_u && !h->seg.has_min && !fix && h->world == 1;
             LeadNSegs lsg{nullptr, nullptr, nullptr, nullptr, 0u, nullptr, nullptr, 1u, h->minq};
             if (lead_n_regions) lsg = LeadNSegs{h->seg.s.as<uint64_t>(), h->seg.e.as<uint64_t>(), h->seg.pmax.as<uint64_t>(), h->seg.id.as<uint32_t>(), h->seg.n, h->seg.reads.as<uint32_t>(), h->seg.mbases.as<uint32_t>(),
-                                                (uint32_t)((h->combined || h->hdr.sample_names.size() <= 1) ? 1 : h->hdr.sample_names.size()), h->minq};
+                                                h->S, h->minq};
             CK(h->lead_list.ensure(Rc * 4));
             BD_LAUNCH((unsigned)((R + 255) / 256), 256, 0, sm, k2_lead_n_find)(soa, u0, (uint32_t)R, h->lead_list.as<uint32_t>(), h->scan_stats.as<ScanStats>());
             BD_LAUNCH(32, 128, 0, sm, k2_lead_n_fix)(soa, u0, h->lead_list.as<uint32_t>(), h->scan_stats.as<ScanStats>(), (h->seg.on && !lead_n_regions) ? 1 : 0,
@@ -1070,6 +1095,7 @@ int run_pipeline_body(bdepth* h, RunMode mode, RunOut* ro, Emitter* em) {
         if (ss.lead_n != ~0ull) return fail(h, BDEPTH_ERR_FORMAT, "read #%llu of the batch: its CIGAR begins with N%s (pileup.d:180-189): there is no result to reproduce", ss.lead_n,
                                              h->seg.on ? " -- the reference computes region / window statistics of such a read partly from its CIGAR as written and partly from a cursor that skips the leading N" : " and ends in a match -- the reference's pileup cursor runs past the read's sequence on such a read");
         if (ss.rg_err != ~0ull) return fail(h, BDEPTH_ERR_FORMAT, "error in read #%llu of the batch: its read group is not present in the header", ss.rg_err);
+        if (ss.untagged_elsewhere) h->pass_untagged = true;
         st.n_records_pass += ss.n_pass; st.n_cigar_ops += ss.n_cigar; st.seq_bytes += ss.seq_bytes; st.long_reads += ss.n_long;
         if (ss.n_pass) { shard_min = std::min<uint64_t>(shard_min, ss.min_start); shard_max = std::max<uint64_t>(shard_max, ss.max_end); }
         if (mode == RUN_SCAN_ONLY) {
@@ -1138,6 +1164,7 @@ int run_pipeline_body(bdepth* h, RunMode mode, RunOut* ro, Emitter* em) {
             BD_LAUNCH((unsigned)((R + 255) / 256), 256, 0, sm, k3_tile_index)(soa, (uint32_t)R, tiles_base, (uint32_t)n_tiles, h->tile_first.as<uint32_t>(), h->tile_lo.as<uint32_t>());
             CK(cudaGetLastError()); st.gpu_launches += 2;
             for (uint32_t si = 0; si < h->S; si++) {      // one counter set per sample (one pass when combined / single sample)
+                if (h->pass_n && rgt.n_rg && !((ss.seen_samples >> si) & 1ull)) continue;      // a sample pass: only the samples this sub-batch holds reads of
                 uint32_t* cnt = h->counts.as<uint32_t>() + (uint64_t)si * N_PLANES * h->win_len; int sel = h->S > 1 ? (int)si : -1;
                 if (ss.n_long) {
                     if (h->minq) BD_LAUNCH((unsigned)((ss.n_long * 32 + 255) / 256), 256, 0, sm, k3_scatter_long<true>)(soa, u0, h->long_list.as<uint32_t>(), (uint32_t)ss.n_long, h->cnt_base, h->win_len, cnt, h->minq, sel);
@@ -1286,9 +1313,32 @@ void add_stats(bdepth_stats& t, const bdepth_stats& s) {
     t.n_cigar_ops += s.n_cigar_ops; t.seq_bytes += s.seq_bytes; t.long_reads += s.long_reads; t.chain_fixups += s.chain_fixups; t.gpu_launches += s.gpu_launches; t.n_batches += s.n_batches;
     t.ms_h2d += s.ms_h2d; t.ms_inflate += s.ms_inflate; t.ms_scan += s.ms_scan; t.ms_coverage += s.ms_coverage; t.ms_span_device += s.ms_span_device; t.host_wall_ms += s.host_wall_ms;
 }
+// One pass of a region / window run whose samples are counted a group at a time (run_segments; the group is h->pass_g0 / pass_n).
+// It reads the inputs whose @RG samples meet the group, and -- when the group holds sample 0 -- those in which an earlier pass met
+// reads without an RG tag (they belong to sample 0, depth.d:240-250; the pass that holds sample 0 runs last).  Every input's records
+// enter n_records once, in the first pass that reads it.
+struct SamplePass {
+    std::vector<char> counted, untagged;      // per input (0: the handle's own, i: extra[i - 1])
+    bool reads(const bdepth* h, size_t i) const {
+        const BamHeader& hd = h->hdr;
+        if (hd.rg_ids.empty()) return h->pass_g0 == 0;          // no @RG lines: every read is sample 0
+        if (h->pass_g0 == 0 && untagged[i]) return true;
+        for (int s : hd.rg_sample) if ((uint32_t)s - h->pass_g0 < h->pass_n) return true;
+        return false;
+    }
+    void note(bdepth* h, size_t i) {
+        if (counted[i]) h->st.n_records = 0;
+        counted[i] = 1;
+        if (h->pass_untagged) untagged[i] = 1;
+    }
+};
 // The pipeline over every input of the handle, into one set of counters (RUN_FULL).  One input: run_pipeline as it is.
-int run_all_inputs(bdepth* h, Emitter* em = nullptr) {
-    if (h->extra.empty()) return run_pipeline(h, RUN_FULL, nullptr, em);
+int run_all_inputs(bdepth* h, Emitter* em = nullptr, SamplePass* sp = nullptr) {
+    if (h->extra.empty()) {
+        const int rc = run_pipeline(h, RUN_FULL, nullptr, em);
+        if (!rc && sp) sp->note(h, 0);
+        return rc;
+    }
     if (h->fix_mates) return fail(h, BDEPTH_ERR_ARG, "fix-mate-overlaps with several BAM files: not available (mates are paired within one file's stream)");
     if (h->world > 1) return fail(h, BDEPTH_ERR_ARG, "several BAM files on several ranks: not available");
     h->staged = false;
@@ -1303,17 +1353,22 @@ int run_all_inputs(bdepth* h, Emitter* em = nullptr) {
         }
         h->cnt_base = lo / TILE_POS * TILE_POS; h->win_len = ((hi - h->cnt_base + TILE_POS - 1) / TILE_POS + 1) * TILE_POS;
         h->force_window = true;
-        bdepth_stats total{}; int rc = 0;
+        bdepth_stats total{}; int rc = 0; size_t n_run = 0;
+        const SamplePass sp0 = sp ? *sp : SamplePass{};      // (what a second attempt starts from)
         for (size_t i = 0; i <= h->extra.size() && !rc; i++) {
             if (i) swap_inputs(h, h->extra[i - 1]);
-            h->accum = i > 0;
-            rc = run_pipeline(h, RUN_FULL, nullptr, nullptr);       // (delivery starts when every input has been counted)
-            add_stats(total, h->st);
+            if (!sp || sp->reads(h, i)) {
+                h->accum = n_run++ > 0;
+                rc = run_pipeline(h, RUN_FULL, nullptr, nullptr);       // (delivery starts when every input has been counted)
+                if (!rc && sp) sp->note(h, i);
+                add_stats(total, h->st);
+            }
             if (i) swap_inputs(h, h->extra[i - 1]);
         }
         h->accum = false; h->force_window = false;
-        if (rc == RC_RETRY_WINDOW) { if (attempt) return fail(h, BDEPTH_ERR_FORMAT, "read extends past the end of the reference space"); continue; }
+        if (rc == RC_RETRY_WINDOW) { if (attempt) return fail(h, BDEPTH_ERR_FORMAT, "read extends past the end of the reference space"); if (sp) *sp = sp0; continue; }
         if (rc) return rc;
+        if (!n_run) return fail(h, BDEPTH_ERR_ARG, "internal: a sample pass that reads no input");
         total.positions = h->hdr.total_len; total.own_lo = h->own_lo; total.own_hi = h->own_hi;
         h->st = total;
         return 0;
@@ -1419,7 +1474,7 @@ void bdepth_close(bdepth_t* h) {
     h->anchors_idx.release(); h->anchors_val.release(); h->chunk_limit.release(); h->tok.release(); h->lits.release(); h->aux.release(); h->segi.release(); h->littab.release();
     DevBuf* bufs[] = {&h->comp, &h->descs, &h->status, &h->ubuf, &h->chunk_start, &h->entry, &h->exitb, &h->count, &h->slot_base, &h->slots, &h->rec_base, &h->walk_list, &h->soa_start, &h->soa_span, &h->soa_meta, &h->soa_off, &h->soa_ncl, &h->soa_lseq, &h->long_list, &h->tile_first, &h->tile_lo, &h->counts, &h->ref_len_d, &h->ref_lin0_d, &h->scan_stats, &h->ref_has, &h->ref_has_all, &h->flt_d, &h->lead_list, &h->misc};
     for (DevBuf* b : bufs) b->release();
-    h->rg_ids.release(); h->rg_offs.release(); h->rg_samp.release();
+    h->rg_ids.release(); h->rg_offs.release(); h->rg_samp.release(); h->rg_hash.release(); h->rg_tab.release();
     h->text[0].release(); h->text[1].release(); h->text_tiles.release(); h->text_offs.release(); h->text_zero.release(); h->text_samp.release(); h->present.release();
     h->seg.s.release(); h->seg.e.release(); h->seg.pmax.release(); h->seg.id.release(); h->seg.reads.release(); h->seg.minstart.release(); h->seg.bases_reads.release(); h->seg.mbases.release(); h->seg.ustart.release(); h->seg.dscr.release(); h->seg.da.release(); h->seg.dac.release(); h->seg.db.release(); h->seg.dthr.release(); h->seg.dbases.release(); h->seg.dcov.release();
     { auto& X = h->ix; X.lin.release(); X.lin_len.release(); X.lin_base.release(); X.lin_cap.release(); X.n_mapped.release(); X.n_unmapped.release(); X.carry.release(); X.ctl.release(); X.runs.release(); X.excs.release(); }
@@ -1458,6 +1513,7 @@ int bdepth_set_filter_query(bdepth_t* h, const char* query) {
     return 0;
 }
 int bdepth_set_combined(bdepth_t* h, int combined) { h->combined = combined != 0; return 0; }
+int bdepth_set_samples_per_pass(bdepth_t* h, uint32_t n) { h->samples_per_pass = n; return 0; }
 int bdepth_set_fix_mates(bdepth_t* h, int on) { if (h->fix_mates != (on != 0)) h->shard_ready = false; h->fix_mates = on != 0; return 0; }      // (with -m a shard is read with zones around it)
 int bdepth_set_min_baseq(bdepth_t* h, uint32_t q) { h->minq = q > 255 ? 255 : q; return 0; }
 int bdepth_set_regions(bdepth_t* h, const bdepth_region* r, size_t n) { normalize_regions(h, r, n, h->regions); return 0; }
@@ -1697,8 +1753,40 @@ int bdepth_run_base_text(bdepth_t* h, const bdepth_text_opts* o, bdepth_text_cb 
     return 0;
 }
 
+// How many samples one pass of a region / window run counts: at most 64 (the sample field of RecordSoA.meta), at most what the
+// counter window leaves room for in HBM (the arithmetic of the check in run_pipeline_body), at most bdepth_set_samples_per_pass.
+// Several ranks take the smallest answer of any of them, so that their passes -- and the collectives inside -- line up.
+static int pass_group_size(bdepth* h, size_t NS, uint32_t& G) {
+    const uint32_t cap = h->samples_per_pass ? std::min<uint32_t>(h->samples_per_pass, 64) : 64;
+    G = cap;
+    const bool shared = h->world > 1 && h->comm;
+    if (NS <= 1 || (shared && NS <= cap)) return 0;      // (several ranks: decided from what they all know)
+    // the counter window as run_all_inputs takes it, the union of what the inputs' indices say: no smaller than any rank's own
+    uint64_t lo = UINT64_MAX, hi = 0;
+    for (size_t i = 0; i <= h->extra.size(); i++) {
+        if (i) swap_inputs(h, h->extra[i - 1]);
+        uint64_t a, b; index_extent(h, a, b); lo = std::min(lo, a); hi = std::max(hi, b);
+        if (i) swap_inputs(h, h->extra[i - 1]);
+    }
+    const uint64_t base = lo / TILE_POS * TILE_POS, win = ((hi - base + TILE_POS - 1) / TILE_POS + 1) * TILE_POS;
+    size_t free_b = 0, tot_b = 0; CK(cudaMemGetInfo(&free_b, &tot_b));
+    const uint64_t fit = (free_b + h->counts.cap) / (win * N_PLANES * 4);
+    G = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(G, fit));      // (nothing fits: one sample, refused by the check itself)
+    if (shared) {
+        cudaStream_t sm = h->s_main; DevBuf mine, all; CK(mine.ensure(16)); CK(all.ensure(16 * (size_t)h->world));
+        CK(cudaMemcpyAsync(mine.p, &G, 4, cudaMemcpyHostToDevice, sm));
+        NK(nccl().AllGather(mine.p, all.p, 1, NCCL_UINT32, h->comm, sm));
+        std::vector<uint32_t> v((size_t)h->world); CK(cudaMemcpyAsync(v.data(), all.p, 4 * (size_t)h->world, cudaMemcpyDeviceToHost, sm)); CK(cudaStreamSynchronize(sm));
+        G = *std::min_element(v.begin(), v.end());
+        mine.release(); all.release();
+    }
+    return 0;
+}
+
 // Shared by window and region modes.  segs: output-order list of (ref, start, end) with end possibly
 // past the reference end (windows); stats are computed over the part inside the reference.
+// Results are laid out [sample][segment].  When the samples' counters do not fit at once (more than 64 samples, HBM, or
+// bdepth_set_samples_per_pass), the pipeline runs once per group of samples and each pass fills its samples' part.
 struct SegDef { uint32_t ref, start, end; uint32_t cov_ext = 0;  /* thresholds are counted from start - cov_ext */ uint32_t min_read_start = 0;  /* != 0: only reads starting at/after it count (quirk 6) */ };
 static int run_segments(bdepth* h, const std::vector<SegDef>& segs, const uint32_t* thr, size_t n_thr,
                         std::vector<uint32_t>& reads, std::vector<uint32_t>& bases, std::vector<uint32_t>& cov) {
@@ -1706,6 +1794,9 @@ static int run_segments(bdepth* h, const std::vector<SegDef>& segs, const uint32
     const size_t n = segs.size();
     const size_t NS = (h->combined || h->hdr.sample_names.size() <= 1) ? 1 : h->hdr.sample_names.size();   // layout: [sample][..]
     const size_t nt1 = std::max<size_t>(n_thr, 1);
+    uint32_t G = 0; rc = pass_group_size(h, NS, G); if (rc) return rc;
+    const size_t n_pass = (NS + G - 1) / G, PS = n_pass > 1 ? G : NS;      // PS: counter sets on the device at once
+    if (n_pass > 1 && h->fix_mates) return fail(h, BDEPTH_ERR_ARG, "fix-mate-overlaps counts every sample in one pass: %zu samples need %zu passes of at most %u samples (use --combined)", NS, n_pass, G);
     reads.assign(NS * n, 0); bases.assign(NS * n, 0); cov.assign(NS * n * nt1, 0);
     // linear-coordinate segments, clipped to the reference
     std::vector<uint64_t> a(n), b(n);
@@ -1728,38 +1819,44 @@ static int run_segments(bdepth* h, const std::vector<SegDef>& segs, const uint32
     }
     auto& S = h->seg;
     size_t nn = n ? n : 1;
-    CK(S.s.ensure(nn * 8)); CK(S.e.ensure(nn * 8)); CK(S.pmax.ensure(nn * 8)); CK(S.id.ensure(nn * 4)); CK(S.reads.ensure(NS * nn * 4)); CK(S.minstart.ensure(nn * 8)); CK(S.bases_reads.ensure(NS * nn * 4)); CK(S.mbases.ensure(NS * nn * 4));
+    CK(S.s.ensure(nn * 8)); CK(S.e.ensure(nn * 8)); CK(S.pmax.ensure(nn * 8)); CK(S.id.ensure(nn * 4)); CK(S.reads.ensure(PS * nn * 4)); CK(S.minstart.ensure(nn * 8)); CK(S.bases_reads.ensure(PS * nn * 4)); CK(S.mbases.ensure(PS * nn * 4));
     if (n) {
         CK(cudaMemcpy(S.s.p, ss.data(), n * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(S.e.p, se.data(), n * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(S.pmax.p, pm.data(), n * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(S.id.p, order.data(), n * 4, cudaMemcpyHostToDevice));
     }
-    CK(cudaMemset(S.reads.p, 0, NS * nn * 4)); CK(cudaMemset(S.bases_reads.p, 0, NS * nn * 4)); CK(cudaMemset(S.mbases.p, 0, NS * nn * 4));
     if (n) CK(cudaMemcpy(S.minstart.p, ms.data(), n * 8, cudaMemcpyHostToDevice));
     CK(S.ustart.ensure(nn * 8)); if (n) CK(cudaMemcpy(S.ustart.p, us.data(), n * 8, cudaMemcpyHostToDevice));
-    CK(S.da.ensure(nn * 8)); CK(S.dac.ensure(nn * 8)); CK(S.db.ensure(nn * 8)); CK(S.dthr.ensure(std::max<size_t>(64, n_thr * 4))); if (n_thr > 16) CK(S.dscr.ensure(NS * nn * 4)); CK(S.dbases.ensure(NS * nn * 4)); CK(S.dcov.ensure(NS * nn * 4 * nt1));
+    CK(S.da.ensure(nn * 8)); CK(S.dac.ensure(nn * 8)); CK(S.db.ensure(nn * 8)); CK(S.dthr.ensure(std::max<size_t>(64, n_thr * 4))); if (n_thr > 16) CK(S.dscr.ensure(PS * nn * 4)); CK(S.dbases.ensure(PS * nn * 4)); CK(S.dcov.ensure(PS * nn * 4 * nt1));
     S.has_min = has_min; S.has_u = has_u; S.ext_max = ext_max;
+    SamplePass spass; spass.counted.assign(h->extra.size() + 1, 0); spass.untagged.assign(h->extra.size() + 1, 0);
+    bdepth_stats total{}; float ms_reduce = 0, ms_exchange = 0; std::vector<uint32_t> has_union;
+    std::vector<uint64_t> wa(n), wb(n), acv(n);      // window-relative segment bounds of a pass (allocated here: not between the device events of the reduction)
+    for (size_t pi = 0; pi < n_pass; pi++) {
+    const size_t g0 = n_pass > 1 ? (pi + 1) % n_pass * G : 0, gn = std::min(PS, NS - g0);      // (the group that holds sample 0 runs last: SamplePass)
+    h->pass_g0 = (uint32_t)g0; h->pass_n = n_pass > 1 ? (uint32_t)gn : 0;
+    CK(cudaMemset(S.reads.p, 0, PS * nn * 4)); CK(cudaMemset(S.bases_reads.p, 0, PS * nn * 4)); CK(cudaMemset(S.mbases.p, 0, PS * nn * 4));
     S.on = true; S.n = (uint32_t)n;
-    rc = run_all_inputs(h);
-    S.on = false;
+    rc = run_all_inputs(h, nullptr, n_pass > 1 ? &spass : nullptr);
+    S.on = false; h->pass_g0 = h->pass_n = 0;
     if (rc) return rc;
     cudaStream_t sm = h->s_main;
     cudaEvent_t e0 = h->ev[5], e1 = h->ev[6];
     CK(cudaEventRecord(e0, sm));
     // per-segment sums over the counters (original order)
     DevBuf &da = S.da, &dac = S.dac, &db = S.db, &dthr = S.dthr, &dbases = S.dbases, &dcov = S.dcov;      // the handle's (sized before the pipeline ran, released with it): no allocation per call
-    std::vector<uint64_t> acv(n); std::vector<uint32_t> qbases, mbases;
+    std::vector<uint32_t> qbases, mbases;
     for (size_t i = 0; i < n; i++) {
         uint64_t lo = std::max(h->cnt_base, h->own_lo), hi = std::min(h->cnt_base + h->win_len, h->own_hi); if (hi < lo) hi = lo;
         uint64_t sc = segs[i].start - std::min(segs[i].cov_ext, segs[i].start);
         uint64_t acov = h->hdr.ref_lin0[segs[i].ref] + std::min<uint64_t>(sc, h->hdr.ref_len[segs[i].ref]);
-        uint64_t wa = std::min(std::max(a[i], lo), hi), wb = std::min(std::max(b[i], lo), hi), wc = std::min(std::max(acov, lo), hi);
-        a[i] = wa - h->cnt_base; b[i] = wb - h->cnt_base; acv[i] = wc - h->cnt_base;
+        uint64_t xa = std::min(std::max(a[i], lo), hi), xb = std::min(std::max(b[i], lo), hi), xc = std::min(std::max(acov, lo), hi);
+        wa[i] = xa - h->cnt_base; wb[i] = xb - h->cnt_base; acv[i] = xc - h->cnt_base;
     }
-    if (n) { CK(cudaMemcpyAsync(da.p, a.data(), n * 8, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(dac.p, acv.data(), n * 8, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(db.p, b.data(), n * 8, cudaMemcpyHostToDevice, sm)); }
+    if (n) { CK(cudaMemcpyAsync(da.p, wa.data(), n * 8, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(dac.p, acv.data(), n * 8, cudaMemcpyHostToDevice, sm)); CK(cudaMemcpyAsync(db.p, wb.data(), n * 8, cudaMemcpyHostToDevice, sm)); }
     if (n_thr) CK(cudaMemcpyAsync(dthr.p, thr, n_thr * 4, cudaMemcpyHostToDevice, sm));
-    CK(cudaMemsetAsync(dbases.p, 0, NS * nn * 4, sm)); CK(cudaMemsetAsync(dcov.p, 0, NS * nn * 4 * nt1, sm));
+    CK(cudaMemsetAsync(dbases.p, 0, PS * nn * 4, sm)); CK(cudaMemsetAsync(dcov.p, 0, PS * nn * 4 * nt1, sm));
     if (n) {
-        for (size_t si = 0; si < NS; si++) {
+        for (size_t si = 0; si < gn; si++) {
             // the kernel keeps 16 threshold counters in registers: more thresholds (the reference has no limit) take further passes over the segments,
             // whose base sums go to a scratch array (they were added by the first pass)
             for (size_t t0 = 0; t0 < std::max<size_t>(n_thr, 1); t0 += 16) {
@@ -1771,24 +1868,36 @@ static int run_segments(bdepth* h, const std::vector<SegDef>& segs, const uint32
         }
         if (h->world > 1 && h->comm) {   // per-segment partial sums are additive over ranks; a failed collective is an error, never a partial sum handed out as the result
             NcclApi& N = nccl();
-            NK(N.AllReduce(dbases.p, dbases.p, NS * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
-            if (n_thr) NK(N.AllReduce(dcov.p, dcov.p, NS * n * n_thr, NCCL_UINT32, NCCL_SUM, h->comm, sm));
-            NK(N.AllReduce(S.reads.p, S.reads.p, NS * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
-            if (has_min) NK(N.AllReduce(S.bases_reads.p, S.bases_reads.p, NS * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
-            if (h->fix_mates) NK(N.AllReduce(S.mbases.p, S.mbases.p, NS * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
+            NK(N.AllReduce(dbases.p, dbases.p, gn * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
+            if (n_thr) NK(N.AllReduce(dcov.p, dcov.p, gn * n * n_thr, NCCL_UINT32, NCCL_SUM, h->comm, sm));
+            NK(N.AllReduce(S.reads.p, S.reads.p, gn * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
+            if (has_min) NK(N.AllReduce(S.bases_reads.p, S.bases_reads.p, gn * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
+            if (h->fix_mates) NK(N.AllReduce(S.mbases.p, S.mbases.p, gn * n, NCCL_UINT32, NCCL_SUM, h->comm, sm));
         }
-        CK(cudaMemcpyAsync(bases.data(), dbases.p, NS * n * 4, cudaMemcpyDeviceToHost, sm));
-        if (n_thr) CK(cudaMemcpyAsync(cov.data(), dcov.p, NS * n * n_thr * 4, cudaMemcpyDeviceToHost, sm));
-        CK(cudaMemcpyAsync(reads.data(), S.reads.p, NS * n * 4, cudaMemcpyDeviceToHost, sm));
-        if (has_min) { qbases.resize(NS * n); CK(cudaMemcpyAsync(qbases.data(), S.bases_reads.p, NS * n * 4, cudaMemcpyDeviceToHost, sm)); }
-        if (h->fix_mates || h->world == 1) { mbases.resize(NS * n); CK(cudaMemcpyAsync(mbases.data(), S.mbases.p, NS * n * 4, cudaMemcpyDeviceToHost, sm)); }      // what n_bases has on top of the base planes: -m (mates.cuh), CIGARs that begin with N (k2_lead_n; zero otherwise)
+        CK(cudaMemcpyAsync(bases.data() + g0 * n, dbases.p, gn * n * 4, cudaMemcpyDeviceToHost, sm));
+        if (n_thr) CK(cudaMemcpyAsync(cov.data() + g0 * n * nt1, dcov.p, gn * n * n_thr * 4, cudaMemcpyDeviceToHost, sm));
+        CK(cudaMemcpyAsync(reads.data() + g0 * n, S.reads.p, gn * n * 4, cudaMemcpyDeviceToHost, sm));
+        if (has_min) { qbases.resize(gn * n); CK(cudaMemcpyAsync(qbases.data(), S.bases_reads.p, gn * n * 4, cudaMemcpyDeviceToHost, sm)); }
+        if (h->fix_mates || h->world == 1) { mbases.resize(gn * n); CK(cudaMemcpyAsync(mbases.data(), S.mbases.p, gn * n * 4, cudaMemcpyDeviceToHost, sm)); }      // what n_bases has on top of the base planes: -m (mates.cuh), CIGARs that begin with N (k2_lead_n; zero otherwise)
     }
     CK(cudaEventRecord(e1, sm));
     CK(cudaStreamSynchronize(sm));
     CK(cudaGetLastError());
-    if (!qbases.empty()) for (size_t si = 0; si < NS; si++) for (size_t i = 0; i < n; i++) if (segs[i].min_read_start) bases[si * n + i] = qbases[si * n + i];
-    if (!mbases.empty()) for (size_t k = 0; k < NS * n; k++) bases[k] += mbases[k];
-    float t = 0; CK(cudaEventElapsedTime(&t, e0, e1)); h->st.ms_reduce = t;
+    if (!qbases.empty()) for (size_t si = 0; si < gn; si++) for (size_t i = 0; i < n; i++) if (segs[i].min_read_start) bases[(g0 + si) * n + i] = qbases[si * n + i];
+    if (!mbases.empty()) for (size_t k = 0; k < gn * n; k++) bases[g0 * n + k] += mbases[k];
+    float t = 0; CK(cudaEventElapsedTime(&t, e0, e1)); ms_reduce += t; ms_exchange += h->st.ms_exchange;
+    if (n_pass > 1) {      // a reference has reads if it has them in any pass
+        add_stats(total, h->st);
+        if (has_union.empty()) has_union = h->ref_has_host; else for (size_t k = 0; k < has_union.size(); k++) has_union[k] |= h->ref_has_host[k];
+    }
+    }   // sample passes
+    if (n_pass > 1) {
+        const bdepth_stats last = h->st;
+        h->st = total; h->st.positions = last.positions; h->st.own_lo = last.own_lo; h->st.own_hi = last.own_hi; h->st.halo_bytes_sent = last.halo_bytes_sent; h->st.ms_exchange = ms_exchange;
+        h->ref_has_host = has_union;
+    }
+    h->st.n_sample_passes = (uint32_t)n_pass;
+    h->st.ms_reduce = ms_reduce;
     h->st.ms_total_device = h->st.ms_h2d + h->st.ms_inflate + h->st.ms_scan + h->st.ms_coverage + h->st.ms_reduce;
     return 0;
 }

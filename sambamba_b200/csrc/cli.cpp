@@ -7,7 +7,9 @@
 // D binding that would replace this file is in sambamba_b200/d/bdepth.d and INTEGRATION.md.
 //
 // Not supported through the GPU path yet (rejected with a message, never silently wrong):
-//   -F with back-references / look-around in regular expressions ; several BAM files together with -m ; more than 64 samples without --combined.
+//   -F with back-references / look-around in regular expressions ; several BAM files together with -m ; `depth base` with more than 64
+//   samples without --combined ; -m in a region / window run whose samples take several passes (more than 64 samples).
+// Region and window modes take any number of samples: the library counts them a group at a time.
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>

@@ -473,39 +473,64 @@ struct ScanStats {      // device-side accumulators
     unsigned long long n_zone_pass, min_start_all;      // several ranks without -m: passing reads of the previous ranks' zone; smallest start over own and zone reads
     unsigned long long lead_n;      // 1 + index of the first read whose CIGAR begins with N and cannot be reproduced (k2_lead_n_fix; ~0: none)
     unsigned long long n_lead;      // reads whose first reference-consuming operation is N (k2_lead_n_find's list)
+    unsigned long long seen_samples;        // RG lookup on: bit s set iff a passing read of pass-local sample s was seen (K3 runs for those only in a sample pass)
+    unsigned long long untagged_elsewhere;  // RG lookup on: nonzero iff a passing read without an RG tag (sample 0) was left to the pass that holds sample 0
 };
 constexpr uint64_t START_UNPLACED = 0xFFFFFFFFFFFFFFFEull;      // RecordSoA.start of a record without a position on a known reference
 constexpr uint32_t NCL_GHOST = 1u << 31;      // RecordSoA.ncl: a record that is only re-read for the mate kernels and passes the filter (its pass bit is clear)
 constexpr uint32_t NCL_FOREIGN = 1u << 30;    // ... and belongs to another rank's shard (-m on several ranks: the zones left and right of the shard)
-// @RG ID -> sample table (depth.d:1170-1181); ids are NUL-terminated, concatenated.  n_rg == 0 disables the scan.
-struct RgTable { const uint8_t* ids; const uint32_t* offs; const uint8_t* sample_of; uint32_t n_rg; };
+// @RG ID -> sample table of one sample pass (depth.d:1170-1181).  ids: the @RG IDs, NUL-terminated, concatenated (offs: where each
+// begins); hash: open-addressing table of 1 + read-group index (0: empty slot), FNV-1a of the ID, linear probing, mask + 1 slots (a power
+// of two >= 2 n_rg, so a probe always ends); sample_of: the read group's pass-local sample id, or RG_OTHER when its sample is counted
+// in another pass; no_tag: the same for sample 0, which reads without an RG tag belong to.  It lives in device memory: k2_decode takes
+// a pointer to it (nullptr: no lookup, every read is sample 0).
+constexpr uint16_t RG_OTHER = 0xFFFFu;
+struct RgTable { const uint8_t* ids; const uint32_t* offs; const uint16_t* sample_of; const uint32_t* hash; uint32_t mask; uint32_t n_rg; uint32_t no_tag; };
+__host__ __device__ __forceinline__ uint32_t fnv1a_step(uint32_t h, uint8_t c) { return (h ^ c) * 16777619u; }
+constexpr uint32_t FNV1A_INIT = 2166136261u;
 
-// CustomBamRead (depth.d:240-250): linear scan of the aux area for RG:Z (read.d:1070-1087); returns the sample id,
-// 0 when the read has no RG tag, -1 when its read group is not in the header.
-__device__ __forceinline__ int sample_of_record(const RgTable& rg, const uint8_t* aux, const uint8_t* end) {
+// CustomBamRead (depth.d:240-250): scan of the aux area for RG:Z (read.d:1070-1087), the ID hashed while it is walked, then one
+// string compare per probe.  Returns the read's pass-local sample id or RG_OTHER.  A read group that is not in the header is booked
+// in st->rg_err (the run fails; the read counts as sample 0 meanwhile).  Out of line, and only in the k2_decode<.., .., true>
+// instantiations: the kernel of single-sample runs keeps its registers.
+__device__ BD_NOINLINE uint32_t sample_of_record(const RgTable* rgp, const uint8_t* aux, const uint8_t* end, ScanStats* st, uint32_t r) {
+    const RgTable rg = *rgp;
     while (aux + 3 <= end) {
         uint8_t t0 = aux[0], t1 = aux[1], ty = aux[2];
         const uint8_t* v = aux + 3;
         if (t0 == 'R' && t1 == 'G' && ty == 'Z') {
-            for (uint32_t g = 0; g < rg.n_rg; g++) {
-                const uint8_t* id = rg.ids + rg.offs[g]; const uint8_t* q = v; bool eq = true;
-                while (q < end && *q) { if (*id != *q) { eq = false; break; } id++; q++; }
-                if (eq && *id == 0) return rg.sample_of[g];
+            uint32_t hs = FNV1A_INIT; const uint8_t* q = v;
+            while (q < end && *q) { hs = fnv1a_step(hs, *q); q++; }
+            const size_t len = (size_t)(q - v);
+            for (uint32_t k = hs & rg.mask;; k = (k + 1) & rg.mask) {
+                const uint32_t g1 = rg.hash[k];
+                if (!g1) break;
+                const uint8_t* id = rg.ids + rg.offs[g1 - 1]; size_t i = 0;
+                while (i < len && id[i] == v[i]) i++;
+                if (i == len && id[len] == 0) {
+                    const uint32_t s = rg.sample_of[g1 - 1];
+                    if (s != RG_OTHER && !((st->seen_samples >> s) & 1ull)) atomicOr(&st->seen_samples, 1ull << s);
+                    return s;
+                }
             }
-            return -1;
+            atomicMin(&st->rg_err, (unsigned long long)r + 1);
+            return rg.no_tag == RG_OTHER ? 0u : rg.no_tag;
         }
-        size_t n;
+        size_t n = 0;
         switch (ty) {
         case 'A': case 'c': case 'C': n = 1; break;
         case 's': case 'S': n = 2; break;
         case 'i': case 'I': case 'f': n = 4; break;
         case 'Z': case 'H': { const uint8_t* q = v; while (q < end && *q) q++; n = (size_t)(q - v) + 1; break; }
-        case 'B': { if (v + 5 > end) return 0; uint8_t st = v[0]; uint32_t cnt = ldu32(v + 1); size_t es = (st == 'c' || st == 'C') ? 1 : (st == 's' || st == 'S') ? 2 : 4; n = 5 + es * cnt; break; }
-        default: return 0;
+        case 'B': { if (v + 5 > end) { aux = end; continue; } uint8_t bt = v[0]; uint32_t cnt = ldu32(v + 1); size_t es = (bt == 'c' || bt == 'C') ? 1 : (bt == 's' || bt == 'S') ? 2 : 4; n = 5 + es * cnt; break; }
+        default: aux = end; continue;      // (an unknown type ends the scan: no RG tag)
         }
         aux = v + n;
     }
-    return 0;
+    // no RG tag: sample 0
+    if (rg.no_tag == RG_OTHER) { if (!st->untagged_elsewhere) atomicExch(&st->untagged_elsewhere, 1ull); }
+    else if (!((st->seen_samples >> rg.no_tag) & 1ull)) atomicOr(&st->seen_samples, 1ull << rg.no_tag);
+    return rg.no_tag;
 }
 
 __device__ __forceinline__ bool cig_rcons(uint32_t op) { return op == 0 || op == 2 || op == 3 || op == 7 || op == 8; }
@@ -516,15 +541,16 @@ __device__ __forceinline__ bool cig_match(uint32_t op) { return op == 0 || op ==
 __device__ BD_NOINLINE bool filter_eval_cold(const FilterProg* fp, const uint8_t* rec, uint32_t rec_size) { return filter_eval(*fp, rec, rec_size); }
 
 // FILTER: a compiled -F query decides (its own instantiation, so that the default predicate's kernel keeps its register count).
+// RG: per-sample counters -- the read's @RG sample is looked up (sample_of_record; rg: the table of the run or sample pass).
 // GHOST (-m across batches and ranks, mates.cuh): records that start below ghost_below were counted by the previous batch,
 // records outside [own_lo, own_hi) belong to a neighbouring rank's shard; both are read only so that the mate kernels see
 // them: their pass bit stays clear (K3, the per-read reducers and the statistics ignore them), NCL_GHOST marks the ones
 // that pass the filter, NCL_FOREIGN the ones of another rank.
-template <bool FILTER, bool GHOST>
+template <bool FILTER, bool GHOST, bool RG>
 __global__ void k2_decode(ScanParams sp, const int64_t* __restrict__ chunk_start, uint32_t n_chunks, const uint32_t* __restrict__ slot_base,
                           const uint16_t* __restrict__ slots, const uint32_t* __restrict__ count, const uint32_t* __restrict__ rec_base,
                           RecordSoA soa, int mapq_gt, uint32_t flag_reject, ScanStats* __restrict__ st, uint32_t* __restrict__ long_list,
-                          uint32_t* __restrict__ ref_has_reads, RgTable rg, const FilterProg* __restrict__ fprog /* compiled -F query, or nullptr: mapq_gt / flag_reject */,
+                          uint32_t* __restrict__ ref_has_reads, const RgTable* __restrict__ rg, const FilterProg* __restrict__ fprog /* compiled -F query, or nullptr: mapq_gt / flag_reject */,
                           int64_t ghost_below, int64_t own_lo, int64_t own_hi, int64_t zone_below /* several ranks without -m: records below this offset
                           belong to the previous ranks' shards and are read only because they reach into this rank's positions: counted by K3, kept out of the statistics */) {
     uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -569,11 +595,11 @@ __global__ void k2_decode(ScanParams sp, const int64_t* __restrict__ chunk_start
         bool is_long = pass && span_eff > SPAN_SHORT;
         uint32_t r = rb + k;
         uint32_t sample = 0;
-        if (rg.n_rg && pass) {
+        if (RG && pass) {
             uint32_t bs = ldu32(sp.u + o);
-            int sid = sample_of_record(rg, cg + 4u * n_cigar + ((uint32_t)l_seq + 1) / 2 + (uint32_t)l_seq, p + bs);
-            if (sid < 0) { atomicMin(&st->rg_err, (unsigned long long)r + 1); sid = 0; }
-            sample = (uint32_t)sid & 63u;
+            const uint32_t sid = sample_of_record(rg, cg + 4u * n_cigar + ((uint32_t)l_seq + 1) / 2 + (uint32_t)l_seq, p + bs, st, r);
+            if (sid == RG_OTHER) { pass = false; is_long = false; }      // counted in the pass that holds its sample
+            else sample = sid & 63u;
         }
         uint32_t ghost_bit = 0;
         if (GHOST) {

@@ -15,6 +15,11 @@
  *
  * usage: bamgen -o out.bam [-n reads] [-s seed] [-t threads] [-l level]
  *               [-r name:len]... | --preset chr20|wgs|tiny  [--stored-every K] [--pairs K]
+ *               [--samples K | --sample NAME]
+ *
+ * --samples K: K read groups rgN / SM:SN (N = 1..K); every read's RG:Z is drawn from the seeded generator.
+ * --sample NAME: the one read group is ID:NAME / SM:NAME (files of one cohort, one sample each).
+ * Without either the file has the read group rg1 / S1, byte for byte as before these options existed.
  */
 #define _GNU_SOURCE
 #include <stdint.h>
@@ -77,6 +82,7 @@ typedef struct {
 static inline void put32(uint8_t *p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
 
 static uint64_t g_pairs = 0;
+static uint32_t g_nsamp = 1; static const char *g_sample = NULL;
 static void gen_read(GenJob *j, Rng *r, uint64_t idx) {
     /* stratified-uniform sorted position in usable linear space */
     double x = ((double)idx + rng_u(r)) / (double)j->total_reads * (double)g_G;
@@ -103,8 +109,8 @@ static void gen_read(GenJob *j, Rng *r, uint64_t idx) {
     /* --pairs K: read idx and read idx + K (about K read spacings further along) share a name, like overlapping mates */
     uint64_t name_id = g_pairs ? (idx / (2 * g_pairs)) * g_pairs + (idx % g_pairs) : idx;
     char name[16]; int l_name = snprintf(name, sizeof name, "r%09llu", (unsigned long long)name_id) + 1;
-    static const char RG[] = "RGZrg1"; /* + NUL */
-    size_t rec = 32 + (size_t)l_name + 4 * (size_t)nc + (READ_LEN + 1) / 2 + READ_LEN + 7 + 4 + 4;
+    char rg[80]; int l_rg = g_sample ? snprintf(rg, sizeof rg, "%s", g_sample) : snprintf(rg, sizeof rg, "rg%u", g_nsamp > 1 ? 1 + rng_below(r, g_nsamp) : 1u);
+    size_t rec = 32 + (size_t)l_name + 4 * (size_t)nc + (READ_LEN + 1) / 2 + READ_LEN + (size_t)(4 + l_rg) + 4 + 4;
     if (j->len + 4 + rec > j->cap) { j->cap = (j->cap + 4 + rec) * 2; j->buf = realloc(j->buf, j->cap); if (!j->buf) die("oom"); }
     uint8_t *p = j->buf + j->len; size_t start = j->len;
     uint32_t bin = (uint32_t)reg2bin(pos, pos + (int64_t)span);
@@ -120,7 +126,7 @@ static void gen_read(GenJob *j, Rng *r, uint64_t idx) {
     { double un = rng_u(r); int nn = un < 0.8607 ? 0 : un < 0.9899 ? 1 : un < 0.99947 ? 2 : 3; for (int k = 0; k < nn; k++) bases[rng_below(r, READ_LEN)] = 15; }
     for (int k = 0; k < READ_LEN; k += 2) *p++ = (uint8_t)((bases[k] << 4) | (k + 1 < READ_LEN ? bases[k + 1] : 0));
     for (int k = 0; k < READ_LEN; ) { uint64_t q = rng_next(r); for (int t = 0; t < 6 && k < READ_LEN; t++, k++) { *p++ = g_qual_tab[q & 1023]; q >>= 10; } }
-    memcpy(p, RG, 7); p += 7;
+    p[0] = 'R'; p[1] = 'G'; p[2] = 'Z'; memcpy(p + 3, rg, (size_t)l_rg + 1); p += 4 + l_rg;
     p[0] = 'N'; p[1] = 'M'; p[2] = 'C'; p[3] = (uint8_t)rng_below(r, 6); p += 4;
     p[0] = 'A'; p[1] = 'S'; p[2] = 'C'; p[3] = (uint8_t)(100 + rng_below(r, 51)); p += 4;
     j->len = (size_t)(p - j->buf);
@@ -245,9 +251,12 @@ int main(int argc, char **argv) {
         else if (!strcmp(argv[i], "--stored-every") && i + 1 < argc) stored_every = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--pairs") && i + 1 < argc) g_pairs = strtoull(argv[++i], NULL, 10);
         else if (!strcmp(argv[i], "--preset") && i + 1 < argc) preset = argv[++i];
+        else if (!strcmp(argv[i], "--samples") && i + 1 < argc) { g_nsamp = (uint32_t)strtoul(argv[++i], NULL, 10); if (g_nsamp < 1 || g_nsamp > 65534) die("--samples: 1 .. 65534"); }
+        else if (!strcmp(argv[i], "--sample") && i + 1 < argc) { g_sample = argv[++i]; if (!*g_sample || strlen(g_sample) > 64 || strpbrk(g_sample, "\t\n")) die("--sample: a name of 1 .. 64 characters without tabs"); }
         else if (!strcmp(argv[i], "-r") && i + 1 < argc) { char *s = argv[++i], *c = strrchr(s, ':'); if (!c) die("bad -r name:len"); refs = realloc(refs, (nref + 1) * sizeof(Ref)); memset(&refs[nref], 0, sizeof(Ref)); snprintf(refs[nref].name, 64, "%.*s", (int)(c - s), s); refs[nref].len = (uint32_t)strtoul(c + 1, NULL, 10); nref++; }
-        else die("usage: bamgen -o out.bam [-n reads] [-s seed] [-t threads] [-l level] [-r name:len]... [--preset chr20|wgs|tiny] [--stored-every K] [--pairs K]");
+        else die("usage: bamgen -o out.bam [-n reads] [-s seed] [-t threads] [-l level] [-r name:len]... [--preset chr20|wgs|tiny] [--stored-every K] [--pairs K] [--samples K | --sample NAME]");
     }
+    if (g_sample && g_nsamp > 1) die("--sample names the one read group of a file: not with --samples");
     if (!out) die("-o required");
     if (preset && !strcmp(preset, "chr20")) { refs = calloc(1, sizeof(Ref)); strcpy(refs[0].name, "chr20"); refs[0].len = 64444167; nref = 1; if (!n_reads) n_reads = 12888833; }
     else if (preset && !strcmp(preset, "wgs")) { refs = calloc(24, sizeof(Ref)); for (int i = 0; i < 24; i++) { if (i < 22) snprintf(refs[i].name, 64, "chr%d", i + 1); else strcpy(refs[i].name, i == 22 ? "chrX" : "chrY"); refs[i].len = GRCH38[i]; } nref = 24; if (!n_reads) n_reads = 620000000ULL; }
@@ -266,7 +275,13 @@ int main(int argc, char **argv) {
     size_t hcap = 1 << 16, hl = 0; char *text = malloc(hcap);
     hl += snprintf(text + hl, hcap - hl, "@HD\tVN:1.6\tSO:coordinate\n");
     for (int i = 0; i < nref; i++) { if (hcap - hl < 256) { hcap *= 2; text = realloc(text, hcap); } hl += snprintf(text + hl, hcap - hl, "@SQ\tSN:%s\tLN:%u\n", refs[i].name, refs[i].len); }
-    hl += snprintf(text + hl, hcap - hl, "@RG\tID:rg1\tSM:S1\tPL:ILLUMINA\n@PG\tID:bamgen\tPN:bamgen\tCL:seed=%llu\n", (unsigned long long)seed);
+    for (uint32_t k = 1; k <= g_nsamp; k++) {
+        if (hcap - hl < 256) { hcap *= 2; text = realloc(text, hcap); }
+        if (g_sample) hl += snprintf(text + hl, hcap - hl, "@RG\tID:%s\tSM:%s\tPL:ILLUMINA\n", g_sample, g_sample);
+        else hl += snprintf(text + hl, hcap - hl, "@RG\tID:rg%u\tSM:S%u\tPL:ILLUMINA\n", k, k);
+    }
+    if (hcap - hl < 256) { hcap *= 2; text = realloc(text, hcap); }
+    hl += snprintf(text + hl, hcap - hl, "@PG\tID:bamgen\tPN:bamgen\tCL:seed=%llu\n", (unsigned long long)seed);
     size_t hdr_len = 12 + hl; for (int i = 0; i < nref; i++) hdr_len += 8 + strlen(refs[i].name) + 1;
     uint8_t *hdr = malloc(hdr_len), *p = hdr;
     memcpy(p, "BAM\1", 4); put32(p + 4, (uint32_t)hl); memcpy(p + 8, text, hl); p += 8 + hl; put32(p, (uint32_t)nref); p += 4;

@@ -95,10 +95,12 @@ def rand_cigar(rng, max_span):
     return cig
 
 
-def rand_case(rng, d, idx):
+def rand_case(rng, d, idx, n_cohort=0):
     n_ref = rng.choice([1, 1, 2, 3, 4])
     refs = [("r%d" % i, rng.choice([60, 300, 1000, 5000, 20000, 40000, 70000])) for i in range(n_ref)]
     n_samp = rng.choice([0, 0, 1, 2, 3])
+    if n_cohort:        # a cohort of more than 64 samples (region / window runs count them a group at a time)
+        n_samp = n_cohort
     rg = [("g%d" % i, "S%d" % (i if rng.random() < 0.8 else 0)) for i in range(n_samp)] or None
     n_reads = rng.choice([0, 1, 5, 40, 200, 600, 1500])
     dense = rng.random() < 0.5
@@ -248,7 +250,7 @@ def rand_bed(rng, refs, path):
     return path
 
 
-def rand_commands(rng, path, refs, d, has_rg, mates_ok, base_only=False):
+def rand_commands(rng, path, refs, d, has_rg, mates_ok, base_only=False, many=False):
     cmds = []
     for _ in range(rng.choice([3, 5, 8])):
         mode = rng.choice(["base", "base", "region", "window"])
@@ -263,9 +265,9 @@ def rand_commands(rng, path, refs, d, has_rg, mates_ok, base_only=False):
             a += ["-C", rng.choice(["1", "4", "9.5", "30"])]
         if rng.random() < 0.25:
             a += ["-a"]
-        if has_rg and rng.random() < 0.3:
+        if has_rg and rng.random() < 0.3 or many and mode == "base":      # (depth base holds at most 64 samples' counters at once)
             a += ["--combined"]
-        if mates_ok and rng.random() < 0.35 and not (base_only and mode != "base"):      # (CIGARs that begin with N: region / window statistics only without -m ...
+        if mates_ok and not many and rng.random() < 0.35 and not (base_only and mode != "base"):      # (CIGARs that begin with N: region / window statistics only without -m ...
             a += ["-m"]
         if mode == "base":
             if rng.random() < 0.2:
@@ -361,7 +363,11 @@ def one_case(seed, idx, keep):
         fails.append((what, detail))
 
     try:
-        path, refs, reads, rg, lead_n = rand_case(rng, d, idx)
+        # a share of the cases is a cohort of 65..150 samples, drawn apart from rng: the other cases stay the ones earlier campaigns ran
+        rc_ = random.Random("cohort%d:%d" % (seed, idx))
+        n_cohort = rc_.randint(65, 150) if rc_.random() < 0.1 else 0
+        path, refs, reads, rg, lead_n = rand_case(rng, d, idx, n_cohort)
+        many = bool(rg) and len({s for _, s in rg}) > 64
         # ---- index: GPU builder (emulated) vs the oracle's IndexBuilder
         rc, out, err = emul_cli(["index", path])
         if rc != 0:
@@ -405,6 +411,23 @@ def one_case(seed, idx, keep):
             if g.shape != want_c.shape or not np.array_equal(g, want_c):
                 bad = np.argwhere(g != want_c)[:3].tolist() if g.shape == want_c.shape else "shape %s vs %s" % (g.shape, want_c.shape)
                 fail("counters fix=%s tuning=%s minq=%d" % (fix, tuning, minq), str(bad))
+        # ---- samples counted a group at a time: bdepth_set_samples_per_pass 1, 3 and 0 (as many as fit) give the same rows (the command
+        # lines below hold the default against the oracle)
+        if rg and 1 < len({s for _, s in rg}) <= 16 and rc_.random() < 0.5:      # (one pass per sample is for small sample counts: the cohorts run as many passes as they need in the command lines)
+            LEGS["passes"] = LEGS.get("passes", 0) + 1
+            tot = sum(l for _, l in refs)
+            minq = rc_.choice([0, 20])
+            outs = []
+            for k in (1, 3, 0):
+                try:
+                    with sb.BDepth(path) as b:
+                        b.set_samples_per_pass(k)
+                        b.set_min_baseq(minq)
+                        outs.append((b.run_regions([(i, 0, L) for i, (_, L) in enumerate(refs)], [1, 5]), b.run_windows(max(100, tot // 500), 0, [2])))
+                except Exception as e:
+                    outs.append(repr(e)[:200])
+            if not outs[0] == outs[1] == outs[2]:
+                fail("samples per pass 1 / 3 / 0 minq=%d" % minq, str([o if isinstance(o, str) else len(o[0]) for o in outs]))
         # ---- several ranks (threads): the owned counters tile the genome and equal the oracle's; region / window rows equal one rank's
         if len(reads) >= 40 and rng.random() < 0.5:
             world = rng.choice([2, 2, 3, 4])
@@ -506,7 +529,7 @@ def one_case(seed, idx, keep):
                 if rc != 0:
                     fail("multi index rc", err.decode()[-300:])
                 files.append(f)
-            for a in rand_commands(rng, path, refs, d, bool(rg), False, base_only=lead_n)[:3]:
+            for a in rand_commands(rng, path, refs, d, bool(rg), False, base_only=lead_n, many=many)[:3]:
                 LEGS["multi"] = LEGS.get("multi", 0) + 1
                 rc1, o1, e1 = emul_cli(["depth"] + a[:-1] + files)
                 rc2, o2, e2 = helpers.oracle_cli(a)
@@ -529,7 +552,7 @@ def one_case(seed, idx, keep):
                      ("ref_id == 0 and position >= %d" % (refs[0][1] // 3), lambda r: r.ref == 0 and r.pos >= refs[0][1] // 3)]
             qtxt, fn = rng.choice(cands)
             sub = helpers.subset_bam(path, os.path.join(d, "sub.bam"), [bool(fn(r)) for r in recs])
-            for a in rand_commands(rng, path, refs, d, bool(rg), mates_ok, base_only=lead_n)[:3]:
+            for a in rand_commands(rng, path, refs, d, bool(rg), mates_ok, base_only=lead_n, many=many)[:3]:
                 a = [x for i, x in enumerate(a) if not (x == "-F" or (i and a[i - 1] == "-F"))]
                 LEGS["filter"] = LEGS.get("filter", 0) + 1
                 rc1, o1, e1 = emul_cli(["depth"] + a[:-1] + ["-F", qtxt, path])
@@ -538,7 +561,7 @@ def one_case(seed, idx, keep):
                     k = next((i for i in range(min(len(o1), len(o2))) if o1[i] != o2[i]), min(len(o1), len(o2)))
                     fail("filter -F '%s': " % qtxt + " ".join(a), "rc %d vs %d; first difference at byte %d: %r vs %r; stderr %r / %r" % (rc1, rc2, k, o1[max(0, k - 60):k + 60], o2[max(0, k - 60):k + 60], e1[-200:], e2[-200:]))
         # ---- command lines
-        for a in rand_commands(rng, path, refs, d, bool(rg), mates_ok, base_only=lead_n):
+        for a in rand_commands(rng, path, refs, d, bool(rg), mates_ok, base_only=lead_n, many=many):
             LEGS["cli"] = LEGS.get("cli", 0) + 1
             rc1, o1, e1 = emul_cli(["depth"] + a)
             rc2, o2, e2 = helpers.oracle_cli(a)
